@@ -7,7 +7,7 @@ transformers, sampling) -> ``MimiModel.decode`` (8 codes -> PCM).  Sessions are 
 with N GPUs every rank runs a replica with its own shard of sessions (no data-path collective),
 so scaling is weak and ``value`` sums the sessions of all ranks.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--sessions B_per_gpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--sessions B_per_gpu] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definition of every field.
 """
@@ -25,6 +25,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the tree may be read-only: the bench writes nothing into it
 os.environ.setdefault("NO_TORCH_COMPILE", "1")
 
 import torch  # noqa: E402
@@ -421,7 +422,10 @@ def b200_arm(args) -> None:
     kv_fill = MOSHI_7B.context if args.kv_fill < 0 else min(args.kv_fill, MOSHI_7B.context)
 
     # the public per-frame API (host buffers in and out): DialogueService.step -> b200_frame_step; its LMGen / Mimi
-    # streaming handles are the ones the device-resident leg drives directly
+    # streaming handles are the ones the device-resident leg drives directly.  Starting to stream seeds each LM's sampling noise
+    # from torch's global generator, which torch seeds at random per process: seed it so that runs with the same arguments sample
+    # the same tokens.
+    torch.manual_seed(4242 + rank)
     svc = DialogueService(B, lm, mimi, use_sampling=True, temp=0.8, temp_text=0.7, kv_dtype=args.kv_dtype)
     gen = svc.lm_gen
     gen.assume_fill(kv_fill)      # steady state: every session already holds `kv_fill` frames of history
@@ -457,7 +461,7 @@ def b200_arm(args) -> None:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for i in range(args.steps):
-                frame(pcm_dev[i % n_buf], timed_lm=True)
+                last = frame(pcm_dev[i % n_buf], timed_lm=True)
             e1.record()
             torch.cuda.synchronize(device)
             barrier()
@@ -514,6 +518,14 @@ def b200_arm(args) -> None:
                "ms_per_step": r["ms_per_step"]}
     if rank != 0:
         return
+    if args.dump_outputs:
+        # what the caller of the timed frame receives in its last step: tokens [B, 1 + 8, 1] (text, audio) and PCM [B, 1, 1920]
+        import numpy as np
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        toks, pcm_out = last
+        np.save(out_dir / "lm_tokens.npy", toks.cpu().double().numpy())
+        np.save(out_dir / "pcm_out.npy", pcm_out.cpu().float().numpy())
     line = {
         "metric": METRIC, "value": value, "unit": "sessions", "n_gpus": world, "steps": args.steps,
         "warmup": max(args.warmup, 3), "ms_per_step": ms_dev, "higher_is_better": True, "scaling": "weak",
@@ -559,7 +571,15 @@ def main() -> None:
                     help="storage of the temporal KV rings; fp8_e4m3 / int8 are opt-in extensions outside the reference's numerics "
                          "(half the ring, twice the sessions per GPU; logit error in tests/test_gpu_zv_kv_q8.py)")
     ap.add_argument("--quantize", action="store_true", help="BASELINE config 5: int8 (W8A8 QLinear) Moshi 7B instead of bf16")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed frame returned to rank 0's sessions as DIR/lm_tokens.npy "
+                         "(float64) and DIR/pcm_out.npy (float32); inputs are seeded, so with the same arguments and session count "
+                         "two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         reference_arm(args)
     else:

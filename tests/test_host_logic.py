@@ -26,7 +26,7 @@ def test_7b_config_matches_reference_json():
     assert abs(total / 1e9 - 7.688) < 0.01            # SURVEY.md: 7.688 B parameters
 
 
-def test_lm_config_rejects_options_outside_hot_path():
+def test_lm_config_rejects_options_outside_hot_path(golden_dir):
     d = MOSHI_7B.to_reference_kwargs()
     d["depformer_causal"] = True                       # deprecated key is accepted and dropped
     LMConfig.from_dict(d)
@@ -40,14 +40,8 @@ def test_lm_config_rejects_options_outside_hot_path():
         LMConfig.from_dict({**d, "causal": False})
     with pytest.raises(ValueError):
         LMConfig.from_dict({**d, "depformer_context": 4})
-    import json
-    from pathlib import Path
-    ref = Path("/root/reference/configs/moshi_dev_2b.json")
-    two_b = json.loads(ref.read_text()) if ref.exists() else {
-        **d, "dim": 2560, "n_q": 32, "dep_q": 16, "num_heads": 20, "num_layers": 24, "depformer_context": 16,
-        "delays": [0, 0] + [2] * 15 + [0] + [2] * 15,
-        "conditioners": {"description": {"type": "lut", "lut": {"n_bins": 31, "dim": 16, "tokenizer": "noop"}}},
-        "fuser": {"sum": ["description"]}}
+    # the reference's configs/moshi_dev_2b.json, stored unmodified
+    two_b = json.loads((golden_dir / "moshi_dev_2b.json").read_text())
     c2 = LMConfig.from_dict(two_b)                     # configs/moshi_dev_2b.json is inside the family now
     assert (c2.n_q, c2.dep_q, c2.max_delay) == (32, 16, 2) and "description" in c2.conditioners
     assert "conditioners" not in c2.to_reference_kwargs()
